@@ -189,9 +189,9 @@ def run_reference_arm(args):
     rank = int(os.environ.get('RANK', 0))
     if rank != 0:
         return
-    # BASELINE.md section 3: b = 4, 2 warm-up + 3 timed fwd + bwd + Adam steps, median (steps / warmup flags are honoured when they are smaller)
+    # b = 4, median of the timed fwd + bwd + Adam steps (BASELINE.md section 3 runs it with --warmup 2 --steps 3)
     b = 4
-    steps, warm = max(1, min(args.steps, 3)), min(args.warmup, 2)
+    steps, warm = args.steps, args.warmup
     tps, ms, cores = cpu_port_tokens_per_s(b, steps, warm)
     line = dict(impl = 'reference', metric = METRIC, value = tps, unit = 'tokens/s', n_gpus = args.gpus, steps = args.steps, warmup = args.warmup, ms_per_step = ms,
                 higher_is_better = True, scaling = 'weak', vs_baseline = None, dtype = 'f32', data = 'synthetic',
@@ -267,6 +267,35 @@ def log(*a):
     print(f'[bench {time.strftime("%H:%M:%S")}]', *a, file = sys.stderr, flush = True)
 
 
+# --------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_LIMIT = 64 << 20                 # bytes written by --dump-outputs in all
+DUMP_PARAMS = 1 << 21                 # parameter values in the fixed sample (float32 values + float64 updates: 24 MB)
+
+
+def param_sample(model):
+    """the values of a fixed, seeded sample of every parameter element (named_parameters order, identical from run to run), float32 on the host"""
+    import torch
+    flat = torch.cat([p.detach().reshape(-1) for p in model.parameters()])
+    idx = torch.randint(0, flat.numel(), (min(DUMP_PARAMS, flat.numel()),), generator = torch.Generator().manual_seed(0)).sort().values
+    return flat[idx.to(flat.device)].float().cpu().numpy()
+
+
+def write_outputs(out_dir, arrays):
+    """writes every (name, array) as out_dir/<name>.npy (float32 stays float32, everything else becomes float64) while the total stays within DUMP_LIMIT"""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok = True)
+    total = 0
+    for name, a in arrays:
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+        if total + a.nbytes > DUMP_LIMIT:
+            log(f'--dump-outputs: {DUMP_LIMIT >> 20} MB reached, {name} and what follows it not written')
+            return
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+        total += a.nbytes
+    log(f'--dump-outputs: {total / 2 ** 20:.1f} MB written to {out_dir}')
+
+
 def run_b200_arm(args):
     import torch
     import torch.distributed as dist
@@ -334,7 +363,7 @@ def run_b200_arm(args):
         e0.record()
         t_host = time.perf_counter()
         for i in range(steps):
-            fn(i)
+            timed.last = fn(i)
         timed.host_ms = 1e3 * (time.perf_counter() - t_host) / steps      # CPU time to enqueue one step (no sync inside)
         e1.record()
         barrier()
@@ -348,6 +377,8 @@ def run_b200_arm(args):
     for i in range(max(args.warmup, 3 * POOL) if (cfg4 and trainer.cuda_graph) else args.warmup):
         step_resident(i)
         torch.cuda.synchronize(); log('warmup step', i, 'done')
+    dump = args.dump_outputs and rank == 0
+    params_before = param_sample(model) if dump else None
     if sampler: sampler.start()
     l0 = eng.ops.launches
     ms_total = timed(step_resident, args.steps)
@@ -355,6 +386,10 @@ def run_b200_arm(args):
     launches = eng.ops.launches - l0
     if sampler:
         sampler.stop()
+    if dump:                        # before the e2e and profiling steps below train the model further
+        params = param_sample(model)
+        write_outputs(args.dump_outputs, [('loss', timed.last.detach().float().reshape(1).cpu().numpy()), ('params', params),
+                                          ('param_update', params.astype('float64') - params_before)])
     ms_step = ms_total / args.steps
     log('resident ms/step', ms_step)
     value = world * B * SEQ / (ms_step / 1e3)
@@ -556,6 +591,16 @@ def run_sample_many(args):
         e1.record(); torch.cuda.synchronize()
         times_ms.append((1e3 * (time.perf_counter() - t0), e0.elapsed_time(e1)))
     sampler.stop()
+    if args.dump_outputs:
+        # the samples of the last timed call, part by part (text ids, modality latents).  Whole samples only, and as many as fit in DUMP_LIMIT
+        # by a per-sample bound that depends on the arguments alone (prompt modality < 65 rows, the forced modality, max_length float64 text ids),
+        # so that two builds always write the same samples
+        keep = min(len(out), DUMP_LIMIT // (4 * (64 + Lm) * 384 + 8 * max_length))
+        if keep < len(out):
+            log(f'--dump-outputs: the first {keep} of {len(out)} samples')
+        write_outputs(args.dump_outputs, [(f'sample{i:03d}_part{j:02d}_text', p.cpu().numpy()) if torch.is_tensor(p) else
+                                          (f'sample{i:03d}_part{j:02d}_modality{p[0]}', p[1].float().cpu().numpy())
+                                          for i, s_ in enumerate(out[:keep]) for j, p in enumerate(s_)])
     launches = (eng.ops.launches - l0) // args.steps
     # one more (untimed) call with CUDA events around every text loop / modality round: where the wall time goes
     model._sampling_timer = {}
@@ -664,7 +709,15 @@ def main():
     ap.add_argument('--no-cpu-baseline', action = 'store_true')
     ap.add_argument('--dump-launches', default = None, help = 'write the entry points of the profiled step in launch order (JSON) - input of tools/ncu_traffic.py')
     ap.add_argument('--no-graph', action = 'store_true', help = 'eager kernel launches instead of CUDA-graph replay (N = 1)')
+    ap.add_argument('--dump-outputs', default = None, metavar = 'DIR',
+                    help = 'after the timed steps write what they computed as DIR/<name>.npy (at most 64 MB; same arguments, same inputs): train / config4 = '
+                           'loss of the last step, a fixed sample of the parameters after it and their change over the timed steps; sample_many = the samples of the last call '
+                           '(with many prompts only the first ones, as many as --prompts / --max-length allow within 64 MB)')
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the B200 arm')
     if args.impl == 'reference':
         run_reference_arm(args)
     elif args.workload == 'sample_many':

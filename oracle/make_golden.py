@@ -16,9 +16,11 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, 'tests'))
 
 from oracle.reference_loader import load_reference          # noqa: E402
 from transfusion_pytorch_b200 import synth                   # noqa: E402
+from helpers import STATE_DICT_CTORS                         # noqa: E402
 
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 
@@ -53,7 +55,8 @@ def noise_for(rb_like_rows, dl, seed):
     return torch.randn(rb_like_rows, dl, generator = torch.Generator().manual_seed(seed))
 
 
-def run_interleaved(ref, name, ctor, batch, times, seed, subsample_rows = None, keep_hiddens = True):
+def run_interleaved(ref, name, ctor, batch, times, seed, subsample_rows = None, keep_hiddens = True, hidden_stride = 1):
+    """hidden_stride: keep every hidden_stride-th token row of the per-layer hiddens (keeps the fixture under 1 MB)"""
     torch.manual_seed(0)
     model = ref.Transfusion(**ctor, modality_processing = 'flat')
     synth.fill_parameters_(model, seed = seed)
@@ -87,7 +90,9 @@ def run_interleaved(ref, name, ctor, batch, times, seed, subsample_rows = None, 
     else:
         fx['embed'] = embed.clone()
         if keep_hiddens:
-            fx['hiddens'] = [h.detach().clone() for h in hiddens[:-1]]
+            fx['hiddens'] = [h.detach()[:, ::hidden_stride].clone() for h in hiddens[:-1]]
+            if hidden_stride > 1:
+                fx['hidden_stride'] = hidden_stride
     torch.save(compact(fx), os.path.join(GOLDEN, f'{name}.pt'))
     print(f'{name}: loss {loss.item():.6f} text {breakdown.text.item():.6f} flow {[round(f.item(), 6) for f in breakdown.flow]} '
           f'positions[0] {proc.modality_positions[0]} total_tokens {proc.total_tokens}')
@@ -161,16 +166,9 @@ def run_sampling_sized(ref, name, ctor, seed, n_each, mod_len, steps, max_length
     model = ref.Transfusion(**ctor)
     synth.fill_parameters_(model, seed = seed)
     model.eval()
-    g = torch.Generator().manual_seed(1234 + seed)
-    dl = ctor['dim_latent']
-    V = ctor['num_text_tokens']
-    prompts = []
-    for k in range(n_each):
-        prompts.append(torch.randint(0, V, (16,), generator = g))
-        prompts.append((0, torch.randn(int(torch.randint(4, 33, (1,), generator = g)), dl, generator = g)))
-        prompts.append(None)
-        prompts.append([torch.randint(0, V, (8,), generator = g), (0, torch.randn(int(torch.randint(6, 33, (1,), generator = g)), dl, generator = g))])
-    noise = torch.randn(mod_len, dl, generator = g)
+    # the inputs are rebuilt from these arguments by tests/helpers.py:load_golden instead of being stored
+    prompt_args = dict(n_each = n_each, text_vocab = ctor['num_text_tokens'], dim_latent = ctor['dim_latent'], noise_len = mod_len, seed = 1234 + seed)
+    prompts, noise = synth.sampling_prompts(**prompt_args)
     kw = dict(max_length = max_length, text_temperature = 0., cfg_scale = 3., modality_steps = steps, init_modality_noise = noise, return_unprocessed_modalities = True)
     if force:
         kw['force_modality_at_start'] = (0, (mod_len,))
@@ -237,7 +235,7 @@ def run_sampling_sized(ref, name, ctor, seed, n_each, mod_len, steps, max_length
                     cur[i] += 1; pos[i] = 0
         rnd += 1
     assert all(len(margins[i]) == sum(len(r) for r in runs[i]) for i in range(B)), 'schedule replay did not consume every sampled token'
-    fx = dict(name = name, ctor = ctor, seed = seed, prompts = prompts, noise = noise, kw = {k: v for k, v in kw.items() if k != 'init_modality_noise'}, samples = out,
+    fx = dict(name = name, ctor = ctor, seed = seed, prompt_args = prompt_args, kw = {k: v for k, v in kw.items() if k != 'init_modality_noise'}, samples = out,
               generated = [[t for r in runs[i] for t in r] for i in range(B)], margins = margins)
     torch.save(compact(fx), os.path.join(GOLDEN, f'{name}.pt'))
     for i, s in enumerate(out):
@@ -267,11 +265,21 @@ def run_velocity(ref, name, ctor, batch, times, seed, delta = 1e-3):
     print(f'{name}: loss {loss.item():.6f} flow {[round(f.item(), 6) for f in breakdown.flow]} velocity {[round(v.item(), 6) for v in breakdown.velocity]} draws {calls}')
 
 
+def write_state_dict_keys(ref):
+    """the reference's state_dict keys, shapes and dtypes for configs 1, 2 and 4 (the weight interchange contract of tests/test_host_cpu.py)"""
+    import json
+    listing = {name: {k: [list(v.shape), str(v.dtype)] for k, v in ref.Transfusion(**ctor).state_dict().items()} for name, ctor in STATE_DICT_CTORS.items()}
+    with open(os.path.join(GOLDEN, 'state_dict_keys.json'), 'w') as f:
+        json.dump(listing, f, indent = 0, sort_keys = True)
+
+
 def main():
     os.makedirs(GOLDEN, exist_ok = True)
     ref = load_reference()
     only = os.environ.get('GOLDEN_ONLY', '')
 
+    if only in ('', 'state_dict'):
+        write_state_dict_keys(ref)
     if only in ('', 'config5'):
         ctor = dict(num_text_tokens = 256, dim_latent = 384, modality_default_shape = (64,), transformer = dict(dim = 512, depth = 8))
         run_sampling_sized(ref, 'config5_mid', ctor, seed = 21, n_each = 2, mod_len = 64, steps = 8, max_length = 96)
@@ -302,7 +310,7 @@ def main():
         ctor = dict(num_text_tokens = 64, dim_latent = 32, modality_default_shape = (4,), transformer = dict(dim = 128, depth = 4, heads = 2, attn_laser = True, use_value_residual = True))
         batch = synth.small_batch(3, seed = 1, dim_latent = 32, text_vocab = 64)
         times = torch.rand(3, count_modalities(batch), generator = torch.Generator().manual_seed(5))
-        run_interleaved(ref, 'small_laser_vres', ctor, batch, times, seed = 1)
+        run_interleaved(ref, 'small_laser_vres', ctor, batch, times, seed = 1, hidden_stride = 2)
         # model_output_clean (MP.py:100-126): the model predicts the clean modality in model space; times pushed towards 1 so that the eps clamp is exercised
         ctor = dict(num_text_tokens = 64, dim_latent = 32, modality_default_shape = (4,), model_output_clean = True, transformer = dict(dim = 128, depth = 2, heads = 2))
         times = (torch.rand(3, count_modalities(batch), generator = torch.Generator().manual_seed(7)) * 1.2).clamp(max = 0.999)
@@ -333,7 +341,7 @@ def main():
     ctor = dict(num_text_tokens = 64, dim_latent = (32, 16), modality_default_shape = ((4,), (2,)), transformer = dict(dim = 128, depth = 4, heads = 4))
     batch = synth.config4_batch(2, seed = 2, total_len = 300, dims = (32, 16), text_vocab = 64)
     times = torch.rand(2, count_modalities(batch), generator = torch.Generator().manual_seed(6))
-    run_interleaved(ref, 'small_two_modalities', ctor, batch, times, seed = 2)
+    run_interleaved(ref, 'small_two_modalities', ctor, batch, times, seed = 2, hidden_stride = 3)
 
     # (3) config 1: text-only pretrain shape (train_text_only.py), d=128 depth=2 heads=8
     ctor = dict(num_text_tokens = 256, transformer = dict(dim = 128, depth = 2))

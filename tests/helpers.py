@@ -7,9 +7,24 @@ from transfusion_pytorch_b200 import synth
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
+# constructors of the reference state_dict listing golden/state_dict_keys.json (configs 1, 2 and 4)
+STATE_DICT_CTORS = dict(
+    config1 = dict(num_text_tokens = 256, transformer = dict(dim = 128, depth = 2)),
+    config2 = dict(num_text_tokens = 256, dim_latent = 384, modality_default_shape = (256,), transformer = dict(dim = 512, depth = 8)),
+    config4 = dict(num_text_tokens = 256, dim_latent = (384, 192), modality_default_shape = ((4,), (2,)), transformer = dict(dim = 512, depth = 8)))
+
 
 def load_golden(name):
-    return torch.load(os.path.join(GOLDEN, f'{name}.pt'), weights_only = False)
+    fx = torch.load(os.path.join(GOLDEN, f'{name}.pt'), weights_only = False)
+    if 'prompt_args' in fx:                          # seeded sampling inputs are rebuilt rather than stored
+        fx['prompts'], fx['noise'] = synth.sampling_prompts(**fx['prompt_args'])
+    return fx
+
+
+def hidden_rows(fx, n):
+    """(slice of our token rows, number of fixture rows) for a sample of n tokens: fixtures may keep only every `hidden_stride`-th row"""
+    step = fx.get('hidden_stride', 1)
+    return slice(0, n, step), -(-n // step)
 
 
 def golden_inputs(name):

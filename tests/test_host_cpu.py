@@ -124,34 +124,21 @@ def test_validation_errors_match_reference_conventions():
 
 def test_state_dict_interchange_with_the_reference():
     """weight interchange contract (SURVEY.md 8(b)): identical state_dict keys, shapes and dtypes as the reference for configs 1, 2 and 4, checked
-    against the reference itself when it is importable (build container) and against the committed key / shape listing otherwise (GPU box); a reference
-    state_dict loads into this model and vice versa."""
+    against the reference's own listing (tests/golden/state_dict_keys.json, written by oracle/make_golden.py from the reference); a checkpoint with
+    exactly the reference's keys, shapes and dtypes loads strictly into this model."""
     import json
-    listing_path = os.path.join(ROOT, 'tests', 'golden', 'state_dict_keys.json')
-    ctors = dict(
-        config1 = dict(num_text_tokens = 256, transformer = dict(dim = 128, depth = 2)),
-        config2 = dict(num_text_tokens = 256, dim_latent = 384, modality_default_shape = (256,), transformer = dict(dim = 512, depth = 8)),
-        config4 = dict(num_text_tokens = 256, dim_latent = (384, 192), modality_default_shape = ((4,), (2,)), transformer = dict(dim = 512, depth = 8)))
-    from oracle.reference_loader import reference_available, load_reference
-    listing = json.load(open(listing_path)) if os.path.isfile(listing_path) else {}
-    ref = load_reference() if reference_available() else None
-    assert ref is not None or listing, 'neither the reference nor the committed listing is available'
-    for name, ctor in ctors.items():
+    from helpers import STATE_DICT_CTORS
+    listing = json.load(open(os.path.join(ROOT, 'tests', 'golden', 'state_dict_keys.json')))
+    assert sorted(listing) == sorted(STATE_DICT_CTORS)
+    for name, ctor in STATE_DICT_CTORS.items():
         ours = Transfusion(**ctor)
         sd = ours.state_dict()
         mine = {k: [list(v.shape), str(v.dtype)] for k, v in sd.items()}
-        if ref is not None:
-            theirs_model = ref.Transfusion(**ctor)
-            theirs = theirs_model.state_dict()
-            want = {k: [list(v.shape), str(v.dtype)] for k, v in theirs.items()}
-            assert mine == want, (sorted(set(mine) ^ set(want))[:6], name)
-            ours.load_state_dict(theirs)                                      # reference checkpoint -> this model
-            theirs_model.load_state_dict(sd)                                  # and back
-            listing[name] = want
-        else:
-            assert mine == listing[name], name
-    if ref is not None:
-        json.dump(listing, open(listing_path, 'w'), indent = 0, sort_keys = True)
+        want = listing[name]
+        assert mine == want, (sorted(set(mine) ^ set(want))[:6], name)
+        theirs = {k: torch.full(shape, 0.5, dtype = getattr(torch, dtype.split('.')[1])) for k, (shape, dtype) in want.items()}
+        ours.load_state_dict(theirs)                                          # reference-shaped checkpoint -> this model
+        assert all(torch.equal(v, theirs[k]) for k, v in ours.state_dict().items())
     assert len(listing['config2']) == 206 and sum(int(np.prod(v[0])) for k, v in listing['config2'].items() if 'weights' not in k) >= 79_545_712
 
 

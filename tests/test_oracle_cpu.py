@@ -4,7 +4,7 @@ API glue) end to end by injecting the oracle engine - the product itself never s
 import pytest
 import torch
 
-from helpers import load_golden, golden_inputs, golden_noise, grad_fingerprint
+from helpers import load_golden, golden_inputs, golden_noise, grad_fingerprint, hidden_rows
 from transfusion_pytorch_b200 import Transfusion, synth
 from oracle.torch_reference import OracleEngine
 
@@ -46,8 +46,8 @@ def test_oracle_matches_reference_small(name):
     for l, h in enumerate(fx['hiddens']):
         ours = st['hiddens'][l]
         for b in range(rb.B):
-            n = int(rb.seq_lens[b])
-            assert torch.allclose(ours[b, :n], h[b, :n], atol = 2e-4, rtol = 1e-4), f'hidden {l} sample {b}'
+            rows, n = hidden_rows(fx, int(rb.seq_lens[b]))
+            assert torch.allclose(ours[b, rows], h[b, :n], atol = 2e-4, rtol = 1e-4), f'hidden {l} sample {b}'
     loss.backward()
     check_grads(model, fx, 1e-3)
 

@@ -4,7 +4,7 @@ import sys, os, traceback
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import torch
-from helpers import load_golden, golden_inputs, golden_noise, grad_fingerprint, unpack_rows
+from helpers import load_golden, golden_inputs, golden_noise, grad_fingerprint, hidden_rows, unpack_rows
 from transfusion_pytorch_b200 import Transfusion, synth
 
 
@@ -28,17 +28,19 @@ def run(name):
           f'flow {[round(f.item(), 6) for f in bd.flow]} (ref {[round(f.item(), 6) for f in fx["flow_losses"]]})')
     print('   positions equal:', rb.modality_positions == fx['modality_positions'], ' total_tokens', rb.total_tokens, fx['total_tokens'])
     st = model.engine.state
+    def tokens(ours, ref, fx_):
+        """the rows of real tokens of every sample (the padding rows of the reference's batch layout are not ours to match), honouring hidden_stride"""
+        pairs = [(ours[b, rows], ref[b, :n]) for b in range(rb.B) for rows, n in [hidden_rows(fx_, int(rb.seq_lens[b]))]]
+        return torch.cat([o for o, _ in pairs]), torch.cat([r for _, r in pairs])
     if 'hiddens' in fx:
         for l, h in enumerate(fx['hiddens']):
-            ours = unpack_rows(st['hid'][l], rb)
-            n = min(ours.shape[1], h.shape[1])
-            print(f'   hidden[{l}] max-rel {rel(ours[:, :n], h[:, :n])[0]:.3e}  l2-rel {rel(ours[:, :n], h[:, :n])[1]:.3e}')
+            ours, ref = tokens(unpack_rows(st['hid'][l], rb), h, fx)
+            print(f'   hidden[{l}] max-rel {rel(ours, ref)[0]:.3e}  l2-rel {rel(ours, ref)[1]:.3e}')
     emb = unpack_rows(st['out'], rb)
     if 'embed_rows' in fx:
         print('   embed rows rel', rel(emb[:, fx['embed_rows']], fx['embed']))
     else:
-        n = min(emb.shape[1], fx['embed'].shape[1])
-        print('   embed rel', rel(emb[:, :n], fx['embed'][:, :n]))
+        print('   embed rel', rel(*tokens(emb, fx['embed'], {})))
     loss.backward()
     torch.cuda.synchronize()
     fp = grad_fingerprint((n, p.grad) for n, p in model.named_parameters() if p.grad is not None)

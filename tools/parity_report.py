@@ -5,7 +5,7 @@ import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import torch
-from helpers import load_golden, golden_inputs, golden_noise, grad_fingerprint, unpack_rows
+from helpers import load_golden, golden_inputs, golden_noise, grad_fingerprint, hidden_rows, unpack_rows
 from transfusion_pytorch_b200 import Transfusion, synth
 
 def rel(a, b): return abs(a - b) / max(abs(b), 1e-12)
@@ -22,8 +22,8 @@ for name in ('small_one_modality', 'small_two_modalities', 'config2_b2', 'config
         for l, h in enumerate(fx['hiddens']):
             ours = unpack_rows(st['hid'][l].float(), rb)
             for b in range(rb.B):
-                n = int(rb.seq_lens[b])
-                hid_err = max(hid_err, ((ours[b, :n].cpu() - h[b, :n]).abs().max() / h[b, :n].abs().max()).item())
+                rows, n = hidden_rows(fx, int(rb.seq_lens[b]))
+                hid_err = max(hid_err, ((ours[b, rows].cpu() - h[b, :n]).abs().max() / h[b, :n].abs().max()).item())
     loss.backward()
     fp = grad_fingerprint((n, p.grad) for n, p in model.named_parameters() if p.grad is not None)
     gerr = max(max(abs(fp[k]['stats'][2].item() - v['stats'][2].item()), abs(fp[k]['stats'][3].item() - v['stats'][3].item())) / max(v['stats'][3].item(), 1e-12) for k, v in fx['grads'].items())

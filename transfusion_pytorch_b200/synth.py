@@ -121,3 +121,16 @@ def config4_batch(batch: int, seed: int = 0, **kw):
 
 def text_batch(batch: int, seq: int, vocab: int = 256, seed: int = 0) -> torch.Tensor:
     return torch.randint(0, vocab, (batch, seq), generator = _gen(31337 + seed))
+
+
+def sampling_prompts(n_each: int, text_vocab: int, dim_latent: int, noise_len: int, seed: int):
+    """(prompts, init_modality_noise) of the config-5 sampling fixtures: 4 x n_each mixed prompts (raw text / raw modality / None /
+    text + modality) and the initial noise of the decoded modality"""
+    g = _gen(seed)
+    prompts = []
+    for _ in range(n_each):
+        prompts.append(torch.randint(0, text_vocab, (16,), generator = g))
+        prompts.append((0, torch.randn(int(torch.randint(4, 33, (1,), generator = g)), dim_latent, generator = g)))
+        prompts.append(None)
+        prompts.append([torch.randint(0, text_vocab, (8,), generator = g), (0, torch.randn(int(torch.randint(6, 33, (1,), generator = g)), dim_latent, generator = g))])
+    return prompts, torch.randn(noise_len, dim_latent, generator = g)
